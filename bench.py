@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 5 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...          # the reference's CPU path (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR        # also write what the last timed `value` step returned (dump_outputs)
 
 Headline workload = BASELINE.json configs[2] (SURVEY.md §8d config 3): 2048x2048 synthetic images, smallest_size 512 => every
 search evaluates 1 + 4 + 16 = 21 crops; 8 searches run in lock-step, each feeding up to 8 frontier crops into a batch of <= 64
@@ -25,6 +26,7 @@ N > 1 (`value`): searches are sharded over ranks (independent units, weights rep
 over ranks of CUDA-event time, value = crops of all ranks / that time ("weak" scaling).
 """
 import argparse
+import atexit
 import csv
 import glob
 import json
@@ -62,7 +64,14 @@ def parse():
     ap.add_argument("--gemm-l2-hints", type=int, default=-1, help="A/B switch for vsb_gemm_set_l2_hints (-1 = library default)")
     ap.add_argument("--fuse-rope", type=int, default=-1, help="A/B switch for vsb_llama_set_fuse_rope (-1 = library default)")
     ap.add_argument("--depth", type=int, default=2, help="frontier batches in flight (1 = round-1 style synchronous rounds)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0's searches and option scorings) to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be >= 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
 
 
 def peaks():
@@ -113,6 +122,7 @@ class ClockSampler:
                  "clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,"
                  "clocks_event_reasons.sw_power_cap", "--format=csv,noheader,nounits", "-lms", "100"],
                 stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)        # no sampler outlives the run when a step raises before stop()
             threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
@@ -298,21 +308,18 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    vals, secs, desc, cores = [], [], "", 1
-    t_wall = time.perf_counter()
-    for i in range(args.warmup + args.steps):
+    warmup = min(args.warmup, 1)          # one warm-up sample pages the weights in; more would only add minutes of CPU time
+    for _ in range(warmup):
+        cpu_reference_sample(args)
+    vals, secs = [], []
+    for _ in range(args.steps):
         v, s, desc, cores = cpu_reference_sample(args)
-        if i >= min(args.warmup, 1):          # one warm-up sample pages the weights in; more would only burn the time budget
-            vals.append(v)
-            secs.append(s)
-        # keep the whole arm within a few minutes on any host: stop once 200 s of wall clock are spent (a slow box then
-        # reports fewer timed samples; "steps" says how many)
-        if time.perf_counter() - t_wall > 200 and vals:
-            break
+        vals.append(v)
+        secs.append(s)
     v = sum(vals) / len(vals)
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": "crops/s",
-        "n_gpus": args.gpus, "steps": len(vals), "warmup": min(args.warmup, 1), "ms_per_step": 1e3 * sum(secs) / len(secs),
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": warmup, "ms_per_step": 1e3 * sum(secs) / len(secs),
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": reference_config(args),
         "cpu_baseline": {"value": v, "unit": "crops/s", "cores": cores, "kind": "port", "sample": desc},
@@ -331,6 +338,48 @@ def workload_config(args):
             "prefix_cache": ("off" if args.no_prefix_cache else
                              "on: K/V of the 37 constant prompt tokens before <im_start> snapshotted at the first (warm-up) prefill and "
                              "shared by all crops; identical results, see DESIGN.md §3 (--no-prefix-cache recomputes them)")}
+
+
+def dump_outputs(path, results, states, scored):
+    """Write what one step returned to its caller as DIR/<name>.npy (float64; the option losses float32), so that two builds
+    can be compared output for output.  Nothing is padded: every value is one the step computed, or 0 where a flag says so.
+    Per search (S searches):
+      search_final_bbox [S,4], search_detection_result [S,4], search_path_length [S], search_success [S]: the result tuple
+      search_valid_boxes_count [S], and search_valid_boxes [sum of the counts, 4] when it is not empty: all_valid_boxes of
+        the searches that succeeded at their root, concatenated in search order
+    Per expanded node, the search paths concatenated in search order (search_path_nodes [S] nodes per search, N in all):
+      search_path_bbox [N,4], search_path_score [N]: the node and its queue priority (0 for a root, which is never queued)
+      search_path_detected [N]: 1 where the node kept its best detection as a candidate (a node where a search succeeds
+        holds it in search_detection_result instead), with search_path_top_logit [N] and search_path_box [N,4] (crop
+        coordinates) set there and 0 elsewhere
+    Per option scoring (if the step ran one): vqa_option_losses [S,n_options], vqa_choice [S]."""
+    import numpy as np
+
+    def f64(x):
+        return np.asarray(x.tolist() if hasattr(x, "tolist") else x, dtype=np.float64)
+
+    nodes = [node for st in states for node in st.search_path]
+    det = [node.get("temp_detection_result") for node in nodes]
+    valid = [f64(av).reshape(-1, 4) for _, _, _, av in results if av is not None and len(av)]
+    out = {"search_final_bbox": f64([fs["bbox"] for fs, _, _, _ in results]),
+           "search_detection_result": f64([f64(fs["detection_result"]) for fs, _, _, _ in results]),
+           "search_path_length": f64([pl for _, pl, _, _ in results]),
+           "search_success": f64([bool(ok) for _, _, ok, _ in results]),
+           "search_valid_boxes_count": f64([0 if av is None else len(av) for _, _, _, av in results]),
+           "search_path_nodes": f64([len(st.search_path) for st in states]),
+           "search_path_bbox": f64([f64(node["bbox"]) for node in nodes]),
+           "search_path_score": f64([0.0 if node["score"] is None else float(node["score"]) for node in nodes]),
+           "search_path_detected": f64([d is not None for d in det]),
+           "search_path_top_logit": f64([0.0 if d is None else float(d[0]) for d in det]),
+           "search_path_box": f64([np.zeros(4) if d is None else f64(d[1]) for d in det])}
+    if valid:
+        out["search_valid_boxes"] = np.concatenate(valid)
+    if scored is not None:
+        out["vqa_option_losses"] = np.stack([f64(losses) for losses, _ in scored]).astype(np.float32)
+        out["vqa_choice"] = f64([choice for _, choice in scored])
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -460,14 +509,16 @@ def run_b200(args):
             if not resident:
                 vsm.release()          # public path: every search image is uploaded (pinned H2D) inside the step
             results, states = visual_search_many(vsm, jobs, batch_size=args.batch, depth=args.depth, **kw)
-            choices = None
+            choices = scored = None
             if with_vqa:
                 if resident:
                     if state["vqa_resident"] is None:
                         state["vqa_resident"] = stage_vqa(results)
-                    choices = [c for _, c in vqa.engine.option_losses_batch(state["vqa_resident"])]
+                    scored = vqa.engine.option_losses_batch(state["vqa_resident"])
+                    choices = [c for _, c in scored]
                 else:
                     choices = vqa_public(results)
+            state["last"] = (results, states, scored)       # what this step returned, for --dump-outputs
             traj = [[tuple(s["bbox"]) for s in st.search_path] for st in states]
             if state["trajectories"] is None:
                 state["trajectories"] = (traj, choices)
@@ -530,6 +581,8 @@ def run_b200(args):
     launches = _lib.launches - launches0
     gemm_flops, gemm_ms, gemm_n = ops.profile_end()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *st2["last"])
     prefix_rows = engine._P
 
     peak_tf, peak_hbm, peak_src = peaks()

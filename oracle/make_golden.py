@@ -375,6 +375,91 @@ def case_bench_eval():
     print("   ", {t: len(v) for t, v in res.items()}, "samples;", sum(len(r["search_result"]) for v in res.values() for r in v), "search results")
 
 
+def case_host_logic():
+    """the reference's answers to the host-logic checks of tests/test_host_logic_vs_reference.py (box geometry, queue order,
+    prompt strings and token splicing, padding and patch geometry, noun chunks, visualisation files) on that module's
+    inputs; images and files are recorded as SHA-256 digests"""
+    print("[golden] host logic")
+    import tempfile
+    import vstar_bench_eval as E   # the reference modules
+    import visual_search as RVS
+    from LLaVA.llava import conversation as rc_vqa
+    from LLaVA.llava.mm_utils import tokenizer_image_object_token as ref_tok_obj
+    from VisualSearch.model.llava import conversation as rc_vsm
+    from VisualSearch.model.llava.mm_utils import tokenizer_image_token as ref_tok
+    from VisualSearch.utils.utils import expand2square as ref_e2s_vsm
+    from tests import test_host_logic_vs_reference as T
+    from vstar_b200.config import tiny_config
+    from vstar_b200.vsm import SyntheticTokenizer
+    g = {}
+
+    split = T.split_inputs()
+    nwnh = [RVS.split_4subpatches(b) for b in split]
+    subs = [RVS.get_sub_patches(b, nw, nh) for b, (nw, nh) in zip(split, nwnh)]
+    g["split_nwnh"] = np.array(nwnh, dtype=np.int64)
+    g["split_subs"] = np.array([s[0] for s in subs], dtype=np.int64)
+    g["split_strides"] = np.array([s[1:] for s in subs], dtype=np.int64)
+
+    cases = T.refine_inputs()
+    g["refine_bbox"] = np.array([RVS.refine_bbox(list(b), W, H) for W, H, b, c in cases], dtype=np.float64)
+    g["iou"] = np.array([RVS.iou(b, c) for W, H, b, c in cases], dtype=np.float64)
+    g["pop_order"] = np.array([T.pop_order(RVS.Prioritize, s) for s in T.pop_inputs()], dtype=np.int64)
+
+    tok = SyntheticTokenizer(tiny_config())
+    prompts = dict(vsm=[], vqa=[])
+    for q in T.PROMPT_QUESTIONS:
+        conv = rc_vsm.conv_templates["llava_v1"].copy()
+        conv.append_message(conv.roles[0], ("<image>" + "\n" + q).replace("<image>", "<im_start><image><im_end>"))
+        conv.append_message(conv.roles[1], "")
+        w = dict(llava_v1=conv.get_prompt(), ids=ref_tok(conv.get_prompt(), tok, return_tensors="pt").tolist())
+        for use_se in (True, False):
+            c2 = rc_vsm.conv_templates["llava_llama_2"].copy()
+            c2.messages = []
+            p2 = "<image>" + "\n" + q
+            if use_se:
+                p2 = p2.replace("<image>", "<im_start><image><im_end>")
+            c2.append_message(c2.roles[0], p2)
+            c2.append_message(c2.roles[1], "")
+            w[f"llava_llama_2_se{int(use_se)}"] = c2.get_prompt()
+        prompts["vsm"].append(w)
+        per_answer = []
+        for answer in T.VQA_ANSWERS:
+            conv = rc_vqa.conv_templates["v1"].copy()
+            conv.append_message(conv.roles[0], T.VQA_QUESTION.format(q))
+            conv.append_message(conv.roles[1], answer)
+            per_answer.append(dict(prompt=conv.get_prompt(), ids=ref_tok_obj(conv.get_prompt(), tok, -200, return_tensors="pt").tolist()))
+        prompts["vqa"].append(per_answer)
+    g["prompts"] = json.dumps(prompts)
+
+    padding = []
+    for i, (w, h) in enumerate(T.PAD_SIZES):
+        img = T.pad_image(i, w, h)
+        a = ref_e2s_vsm(img, T.PAD_BG)
+        b, left, top = E.expand2square(img, T.PAD_BG)
+        padding.append(dict(vsm=[a.width, a.height, T.image_digest(a)], vqa=[b.width, b.height, T.image_digest(b), left, top]))
+    g["padding"] = json.dumps(padding)
+    g["get_patch"] = np.array([[E.VQA_LLM.get_patch(None, bbox, W, H, patch_scale=s) for s in T.PATCH_SCALES]
+                               for W, H, bbox in T.patch_inputs()], dtype=np.int64)
+
+    nlp = FakeNLP()
+    RVS.nlp = nlp
+    phrases, chunk_lists = T.noun_chunk_inputs()
+    g["noun_chunks"] = json.dumps(dict(
+        chunks=[RVS.extract_noun_chunks(ph) for ph in phrases],
+        spans=[[list(RVS.get_noun_chunks(t)) + list(RVS.tranverse(t)) for t in nlp(ph)] for ph in phrases],
+        filtered=[RVS.filter_chunk_list(c) for c in chunk_lists]))
+
+    vis = []
+    for seed, w, h, smallest, hot, kw in T.VIS_CASES:
+        with tempfile.TemporaryDirectory() as d:
+            r = RVS.visual_search(StubVSM(hot), synth_image(seed, w, h), "mug", T.VIS_TARGET_BBOX, smallest, visualize=True,
+                                  save_path=d, **kw)
+            vis.append(dict(path_length=r[1], success=bool(r[2]), files=T.dir_digests(d)))
+    g["visualisation"] = json.dumps(vis)
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "host_logic.npz"), **g)
+    print("   ", len(split), "boxes,", len(phrases), "phrases,", sum(len(v["files"]) for v in vis), "visualisation files")
+
+
 def search_edge_cases():
     """termination / selection branches of visual_search() (visual_search.py:399-413, :428-431, :497-512)"""
     case_search("edge_root_hit", img_seed=24, w=1280, h=960, smallest=224, hot="root")          # success at the root, 3 valid boxes
@@ -400,6 +485,10 @@ def main():
         assert ref_shims.reference_available()
         ref_shims.install(*hf_cfgs(O.tiny_config()))
         return case_bench_eval()
+    if os.environ.get("GOLDEN_ONLY") == "host_logic":
+        assert ref_shims.reference_available()
+        ref_shims.install(*hf_cfgs(O.tiny_config()))
+        return case_host_logic()
     assert ref_shims.reference_available(), "needs /root/reference (build container only)"
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     torch.set_num_threads(8)
@@ -430,6 +519,7 @@ def main():
     search_model_separated(m, sd, cfg)
     case_vqa("a", img_seed=41)
     case_bench_eval()
+    case_host_logic()
     print("golden vectors written to", GOLDEN_DIR)
 
 

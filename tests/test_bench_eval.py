@@ -14,7 +14,9 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden", "bench_eval_golden.json
 
 def run(tmp_path, in_flight, tag):
     from vstar_b200.bench_eval import eval_model
-    folder = make_bench_folder(str(tmp_path / "bench"))
+    # the driver takes an annotation's path to be its image's path up to the first '.' (as the reference does), so the
+    # tree is named relative to tmp_path (the working directory), whose own path may contain dots
+    folder = make_bench_folder("bench")
     out = str(tmp_path / f"out_{tag}.json")
     args = types.SimpleNamespace(benchmark_folder=folder, output_path=out, vsm_model_path="stub", minimum_size_scale=4.0,
                                  minimum_size=224, images_in_flight=in_flight, search_batch=8)
@@ -41,7 +43,8 @@ def check_against_golden(res):
 
 
 @pytest.mark.parametrize("in_flight", [1, 3, 8])
-def test_matches_reference_driver(tmp_path, in_flight):
+def test_matches_reference_driver(tmp_path, monkeypatch, in_flight):
+    monkeypatch.chdir(tmp_path)
     res, overall, dumped, lines = run(tmp_path, in_flight, str(in_flight))
     assert dumped == json.loads(json.dumps(res))
     check_against_golden(dumped)
